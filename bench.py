@@ -15,6 +15,8 @@ per-shard top-k, one merge kernel.
 --impl reference: the CPU arm -- the oracle's restatement of the reference's brute-force path
 (one thread per part, SIMD inner-product blocks; the reference binary cannot be built here,
 see DESIGN.md), timed on a bounded row sample and scaled linearly to the full corpus.
+--dump-outputs DIR: the answer of the last timed step (what a caller of the timed path receives) as DIR/distances.npy
+(float32) and DIR/ids.npy (float64), so that two builds can be compared output for output on identical seeded inputs.
 """
 import argparse
 import json
@@ -26,6 +28,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 # BASELINE.json's metric ("QPS @ recall@10>=0.95 ...") on configs[1]; exact brute force, so recall@10 is 1.0
 METRIC = "QPS @ recall@10>=0.95 (exact: recall 1.0), FLAT brute-force IP top-10, 10M x 768-d bf16, batch 1024"
@@ -52,7 +55,34 @@ def parse():
     ap.add_argument("--headline-only", action="store_true", help="A/B runs: skip verification and the extra keys")
     ap.add_argument("--index-rows", type=int, default=100_000_000, help="rows of the MSTG-class index extra (BASELINE configs[2]); 0 = skip")
     ap.add_argument("--index-nq", type=int, default=256)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's distances and ids as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times the CPU oracle on a row sample)")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, dis, ids):
+    """Writes the top-k answer as float32 distances / float64 ids (exact below 2**53).  Above DUMP_BYTES, a fixed seeded
+    sample of query rows is written, with their indices in query_rows.npy."""
+    import numpy as np
+    nq = dis.shape[0]
+    cap = max(1, DUMP_BYTES // max(1, dis.shape[1] * (4 + 8)))
+    arrays = {}
+    if nq > cap:
+        rows = np.sort(np.random.default_rng(0).choice(nq, size=cap, replace=False))
+        dis, ids = dis[rows], ids[rows]
+        arrays["query_rows"] = rows.astype(np.float64)
+    arrays["distances"] = np.ascontiguousarray(dis, dtype=np.float32)
+    arrays["ids"] = np.ascontiguousarray(ids, dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
 
 
 def config_of(a, n):
@@ -635,6 +665,8 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     launches = S.launch_count()
+    if a.dump_outputs and rank == 0:   # now: the e2e loop and the fp32 extra below reuse these buffers
+        dump_outputs(a.dump_outputs, (o_dis if N == 1 else f_dis).cpu().numpy(), (o_ids if N == 1 else f_ids).cpu().numpy())
     kern_ms, kern_n = index.kernel_time(reset=True)
     clocks = sampler.stop()
     if N > 1:  # kernel time for the roofline: a few eager steps with per-launch events, outside the timed region

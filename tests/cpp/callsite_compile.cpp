@@ -12,6 +12,7 @@
 
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
 #include <filesystem>
 #include <variant>
 
@@ -280,8 +281,10 @@ int main() {
 
         // ---------------- TantivyIndexStore.cpp call sites
         {
-            const String index_files_cache_path = "/tmp/b200_callsite_fts";
-            std::filesystem::create_directories(index_files_cache_path);   // the part's FTS cache directory (index_files_manager)
+            // the part's FTS cache directory (index_files_manager): a fresh one per run, so concurrent runs never share it
+            String fts_dir_template = (std::filesystem::temp_directory_path() / "b200_callsite_fts_XXXXXX").string();
+            REQUIRE(mkdtemp(fts_dir_template.data()) != nullptr);
+            const String index_files_cache_path = fts_dir_template;
             std::vector<String> indexed_columns = {"doc", "title"};
             const String index_json_parameter = "{}";
             TANTIVY::FFIBoolResult create_status = TANTIVY::ffi_create_index_with_parameter(index_files_cache_path, indexed_columns, index_json_parameter);   // :713
@@ -329,7 +332,8 @@ int main() {
             result = TANTIVY::ffi_bm25_search(index_files_cache_path, sentence, column_names, static_cast<uint32_t>(topk), {}, false, enable_nlq, operator_or, statistics);
             REQUIRE(!result.error.is_error && result.result.size() == 3);
             TANTIVY::ffi_free_index_reader(index_files_cache_path);
-            REQUIRE(TANTIVY::ffi_load_index_reader("/tmp/b200_no_such_dir").error.is_error);
+            REQUIRE(TANTIVY::ffi_load_index_reader(index_files_cache_path + "/no_such_dir").error.is_error);
+            std::filesystem::remove_all(index_files_cache_path);
         }
         std::printf("CALLSITES OK\n");
         return 0;
